@@ -2,6 +2,7 @@
 """bench.py -- NEXMark events/sec through the B200-native executor (BASELINE.json metric).
 
     python bench.py --gpus N --steps K --warmup W            # this repo's GPU path
+    python bench.py --gpus 1 ... --dump-outputs DIR          # + the q2 result of the last timed step as DIR/<column>.npy
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port) on host cores
 
 N = 1  headline workload "nexmark_q2_10M_bids" = BASELINE.json configs[1]: NEXMark q2 (SELECT auction, price FROM bid
@@ -55,6 +56,7 @@ EVENTS_PER_GPU = 125_000_000  # BASELINE.json configs[4] / 8
 BATCH_ROWS = 65536
 RING = 4                     # distinct resident relations rotated through (defeats the 126 MB L2)
 UNIT = "events/s"
+DUMP_BYTES = 64_000_000      # --dump-outputs: at most this many bytes of .npy data in all
 
 
 # Libraries write to fd 1 behind Python's back (NCCL prints "NCCL version ..." there): keep the real stdout for the
@@ -301,6 +303,20 @@ def time_plan(ctx, ec, tables, reps: int, dist: Dist | None = None, flush: bool 
     return out, rows, statistics.median(times), min(times), prof, launches
 
 
+def dump_outputs(table: pa.Table, out_dir: str) -> None:
+    """Writes every column of `table` as out_dir/<column>.npy in float64 (exact for the int32 columns of q2), so that two
+    builds can be compared array for array.  Beyond DUMP_BYTES in all, the same fixed, seeded sample of rows (in row
+    order) is taken from every column."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    n, cap = table.num_rows, DUMP_BYTES // (8 * max(table.num_columns, 1))
+    rows = np.sort(np.random.default_rng(0).choice(n, cap, replace=False)) if n > cap else None
+    for name in table.column_names:
+        v = table[name].to_numpy().astype(np.float64)
+        np.save(d / f"{name}.npy", v if rows is None else v[rows])
+    log(f"dumped {table.column_names} of the last timed step ({n} rows{'' if rows is None else f', {cap} sampled'}) to {d}")
+
+
 def dominant(prof: dict) -> tuple[str | None, float]:
     if not prof:
         return None, 0.0
@@ -454,6 +470,7 @@ def run_gpu_q2(args, dist: Dist) -> dict:
     dev_ms = ctx.timer_ms(0)
     launches = ctx.kernel_launches - launches0
     assert keep[-1].num_rows == n_sel[(args.warmup + args.steps - 1) % RING]
+    last_step = keep[-1] if args.dump_outputs else None     # the result of the last step of `value`'s region
     # ---- timed region B: the same K steps again with a CUDA-event pair around every launch (flockgpu_profile_*) -> the
     # kernel's mean duration for `roofline`.  Kept apart from A because the event pairs themselves cost ~3 us per step
     # (27.8 vs 24.4 us per step, runs 28 / 32); `ms_per_step_instrumented` reports B next to A.
@@ -524,6 +541,9 @@ def run_gpu_q2(args, dist: Dist) -> dict:
     e2e = dict(e2e_pageable)
     e2e["variants"] = {"pageable": e2e_pageable, "host_register": e2e_registered, "page_locked_zero_copy": e2e_pinned}
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(last_step.to_arrow(), args.dump_outputs)
+    del last_step
 
     # ---- roofline of the dominant kernel
     peak, peak_src = measured_peak_gbs()
@@ -943,7 +963,13 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=None, help="steps of the host-buffer legs (default: --steps, capped per variant)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-queries", action="store_true", help="skip the `queries` object (q1 / q3 / q5 / q8 on one GPU, q2 on N GPUs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the q2 result of the last timed step as DIR/<column>.npy (float64; seeded sample above 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "gpu" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs applies to the one-GPU q2 run (--impl gpu, one process)")
     if args.impl == "reference":
         res = run_reference(args)
     else:
