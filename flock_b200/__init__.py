@@ -7,7 +7,7 @@ Interface through pyarrow); the product is libflockgpu.so.  Names follow the ref
                                 execute_partitioned / clean_data_sources / is_shuffling)
     Context.filter_project      FilterExec + CoalesceBatchesExec + ProjectionExec
     Context.hash_aggregate      HashAggregateExec {Partial, Final, FinalPartitioned}
-    Context.hash_join           HashJoinExec {Partitioned, Inner}
+    Context.hash_join           HashJoinExec {Partitioned, Inner | Left | Right | Full | Semi | Anti}
     Context.hash_partition      RepartitionExec: Hash(keys, n)
 """
 from __future__ import annotations
@@ -393,11 +393,18 @@ class Context:
         check(lib.flockgpu_hash_aggregate(self.handle, table.handle, m, g, len(group_cols), specs, len(aggs), C.byref(out)))
         return Table(self, out.value)
 
-    def hash_join(self, left: Table, right: Table, left_keys: Sequence[int], right_keys: Sequence[int]) -> Table:
+    def hash_join(self, left: Table, right: Table, left_keys: Sequence[int], right_keys: Sequence[int], join_type: str = "inner") -> Table:
+        """join_type: inner, left, right, full (output left ++ right columns) or semi, anti (left columns only, left order)."""
+        jt = _ffi.JOIN_TYPES.get(join_type.lower()) if isinstance(join_type, str) else None
+        if jt is None:
+            raise ValueError(f"unknown join type {join_type!r}; expected one of {sorted(_ffi.JOIN_TYPES)}")
         lk = (C.c_int32 * len(left_keys))(*left_keys)
         rk = (C.c_int32 * len(right_keys))(*right_keys)
         out = C.c_void_p()
-        check(lib.flockgpu_hash_join(self.handle, left.handle, right.handle, lk, rk, len(left_keys), C.byref(out)))
+        if jt == 0:
+            check(lib.flockgpu_hash_join(self.handle, left.handle, right.handle, lk, rk, len(left_keys), C.byref(out)))
+        else:
+            check(lib.flockgpu_hash_join_typed(self.handle, left.handle, right.handle, lk, rk, len(left_keys), jt, C.byref(out)))
         return Table(self, out.value)
 
     def hash_partition(self, table: Table, key_cols: Sequence[int], n_parts: int) -> list[Table]:

@@ -25,6 +25,9 @@ class FlockGpuError(RuntimeError):
 # error codes (include/flockgpu.h)
 OK, ERR_INVALID, ERR_UNSUPPORTED, ERR_CUDA, ERR_NCCL, ERR_EXECUTION, ERR_NO_DEVICE = 0, -1, -2, -3, -4, -5, -6
 
+# enum flockgpu_join_type, by the lower-case DataFusion 6 JoinType name
+JOIN_TYPES = {"inner": 0, "left": 1, "right": 2, "full": 3, "semi": 4, "anti": 5}
+
 
 class ArrowSchema(C.Structure):
     pass
@@ -143,6 +146,7 @@ PROTOTYPES = {
     "flockgpu_filter_project": (C.c_int, [_P, _P, C.POINTER(Expr), C.POINTER(Expr), C.POINTER(C.c_char_p), C.c_int32, _PP]),
     "flockgpu_hash_aggregate": (C.c_int, [_P, _P, C.c_int32, _I32P, C.c_int32, C.POINTER(AggSpec), C.c_int32, _PP]),
     "flockgpu_hash_join": (C.c_int, [_P, _P, _P, _I32P, _I32P, C.c_int32, _PP]),
+    "flockgpu_hash_join_typed": (C.c_int, [_P, _P, _P, _I32P, _I32P, C.c_int32, C.c_int32, _PP]),
     "flockgpu_hash_partition": (C.c_int, [_P, _P, _I32P, C.c_int32, C.c_int32, _PP]),
     "flockgpu_sort": (C.c_int, [_P, _P, _I32P, _I32P, C.c_int32, _PP]),
     "flockgpu_row_number": (C.c_int, [_P, _P, _I32P, C.c_int32, C.c_char_p, _PP]),

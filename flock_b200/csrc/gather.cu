@@ -46,22 +46,40 @@ struct GatherMultiArgs {
   int32_t width[GM_MAX_COLS];
 };
 
+// PAD: the index may hold the pad sentinel GATHER_PAD (an outer join's unmatched row): its value is 0.  The Inner join
+// and every other take() launch PAD = false, which is the kernel as it was before the sentinel existed.
+constexpr uint32_t GATHER_PAD = ~0u;
+
+template <bool PAD>
 __global__ void __launch_bounds__(GA_THREADS) gather_fixed_multi_kernel(const __grid_constant__ GatherMultiArgs a) {
   const int64_t stride = int64_t(gridDim.x) * GA_THREADS;
   for (int64_t i = int64_t(blockIdx.x) * GA_THREADS + threadIdx.x; i < a.n; i += 2 * stride) {
     const int64_t j = i + stride;
-    const uint32_t r0 = a.idx[i], r1 = j < a.n ? a.idx[j] : 0u;
+    const uint32_t r0 = a.idx[i], r1 = j < a.n ? a.idx[j] : (PAD ? GATHER_PAD : 0u);
     for (int c = 0; c < a.n_cols; ++c) {
       if (a.width[c] == 4) {
-        const uint32_t v0 = static_cast<const uint32_t*>(a.src[c])[r0], v1 = j < a.n ? static_cast<const uint32_t*>(a.src[c])[r1] : 0u;
+        const uint32_t v0 = PAD && r0 == GATHER_PAD ? 0u : static_cast<const uint32_t*>(a.src[c])[r0];
+        const uint32_t v1 = PAD && r1 == GATHER_PAD ? 0u : j < a.n ? static_cast<const uint32_t*>(a.src[c])[r1] : 0u;
         static_cast<uint32_t*>(a.dst[c])[i] = v0;
         if (j < a.n) static_cast<uint32_t*>(a.dst[c])[j] = v1;
       } else {
-        const uint64_t v0 = static_cast<const uint64_t*>(a.src[c])[r0], v1 = j < a.n ? static_cast<const uint64_t*>(a.src[c])[r1] : 0ull;
+        const uint64_t v0 = PAD && r0 == GATHER_PAD ? 0ull : static_cast<const uint64_t*>(a.src[c])[r0];
+        const uint64_t v1 = PAD && r1 == GATHER_PAD ? 0ull : j < a.n ? static_cast<const uint64_t*>(a.src[c])[r1] : 0ull;
         static_cast<uint64_t*>(a.dst[c])[i] = v0;
         if (j < a.n) static_cast<uint64_t*>(a.dst[c])[j] = v1;
       }
     }
+  }
+}
+
+// Validity of a column taken through an index with pad sentinels: 0 for a sentinel, else the source's byte (1 when the
+// source has no validity).
+__global__ void __launch_bounds__(GA_THREADS) gather_valid_pad_kernel(const uint8_t* __restrict__ in, const uint32_t* __restrict__ idx,
+                                                                      uint8_t* __restrict__ out, int64_t n) {
+  const int64_t stride = int64_t(gridDim.x) * GA_THREADS;
+  for (int64_t i = int64_t(blockIdx.x) * GA_THREADS + threadIdx.x; i < n; i += stride) {
+    const uint32_t r = idx[i];
+    out[i] = r == GATHER_PAD ? uint8_t(0) : in ? in[r] : uint8_t(1);
   }
 }
 
@@ -77,6 +95,7 @@ struct GatherLenArgs {
   CompactScratch sc;  // grid-wide exclusive prefix of the tiles' byte counts (compact.cuh); sc.out_count = total bytes
 };
 
+template <bool PAD>
 __global__ void __launch_bounds__(GA_THREADS) gather_lengths_scan_kernel(const __grid_constant__ GatherLenArgs a) {
   __shared__ CompactSmem<1, 16> sm;
   __shared__ unsigned long long s_warp[GA_THREADS / 32];
@@ -91,7 +110,7 @@ __global__ void __launch_bounds__(GA_THREADS) gather_lengths_scan_kernel(const _
       len[k] = 0;
       if (i0 + k < a.n) {
         int64_t r = a.idx ? int64_t(a.idx[i0 + k]) : i0 + k;
-        len[k] = unsigned(a.in_off[r + 1] - a.in_off[r]);
+        if (!PAD || r != int64_t(GATHER_PAD)) len[k] = unsigned(a.in_off[r + 1] - a.in_off[r]);
       }
       local += len[k];
     }
@@ -131,6 +150,7 @@ struct GatherLenMultiArgs {
   CompactScratch sc;           // sc.num_tiles = n_cols * tiles, single wave
 };
 
+template <bool PAD>
 __global__ void __launch_bounds__(GA_THREADS) gather_lengths_scan_multi_kernel(const __grid_constant__ GatherLenMultiArgs a) {
   __shared__ CompactSmem<1, 16> sm;
   __shared__ unsigned long long s_warp[GA_THREADS / 32];
@@ -148,7 +168,7 @@ __global__ void __launch_bounds__(GA_THREADS) gather_lengths_scan_multi_kernel(c
     len[k] = 0;
     if (i0 + k < a.n) {
       const int64_t r = a.idx ? int64_t(a.idx[i0 + k]) : i0 + k;
-      len[k] = unsigned(in_off[r + 1] - in_off[r]);
+      if (!PAD || r != int64_t(GATHER_PAD)) len[k] = unsigned(in_off[r + 1] - in_off[r]);
     }
     local += len[k];
   }
@@ -183,6 +203,7 @@ struct GatherCopyMultiArgs {
 };
 constexpr int GU_STAGE = 2048;  // bytes of shared staging per warp
 
+template <bool PAD>
 __device__ __forceinline__ void gather_utf8_copy_body(const uint8_t* __restrict__ in_data, const int32_t* __restrict__ in_off,
                                                       const uint32_t* __restrict__ idx, const int32_t* __restrict__ out_off,
                                                       uint8_t* __restrict__ out_data, int64_t n) {
@@ -203,7 +224,7 @@ __device__ __forceinline__ void gather_utf8_copy_body(const uint8_t* __restrict_
       dst_start = out_off[r0 + lane];
       len = out_off[r0 + lane + 1] - dst_start;
       int64_t r = idx ? int64_t(idx[r0 + lane]) : r0 + lane;
-      src_start = in_off[r];
+      if (!PAD || r != int64_t(GATHER_PAD)) src_start = in_off[r];  // a padded row has length 0: no byte is read
     }
     const int32_t d0 = __shfl_sync(FULL_MASK, dst_start, 0);
     const int32_t d1 = out_off[r0 + rows];
@@ -247,16 +268,18 @@ __device__ __forceinline__ void gather_utf8_copy_body(const uint8_t* __restrict_
   }
 }
 
+template <bool PAD>
 __global__ void __launch_bounds__(GA_THREADS) gather_utf8_copy_kernel(const uint8_t* __restrict__ in_data, const int32_t* __restrict__ in_off,
                                                                        const uint32_t* __restrict__ idx, const int32_t* __restrict__ out_off,
                                                                        uint8_t* __restrict__ out_data, int64_t n) {
-  gather_utf8_copy_body(in_data, in_off, idx, out_off, out_data, n);
+  gather_utf8_copy_body<PAD>(in_data, in_off, idx, out_off, out_data, n);
 }
 
 // every Utf8 column of a take() in one launch: blockIdx.y = column
+template <bool PAD>
 __global__ void __launch_bounds__(GA_THREADS) gather_utf8_copy_multi_kernel(const __grid_constant__ GatherCopyMultiArgs a) {
   const int c = blockIdx.y;
-  gather_utf8_copy_body(a.in_data[c], a.in_off[c], a.idx, a.out_off[c], a.out_data[c], a.n);
+  gather_utf8_copy_body<PAD>(a.in_data[c], a.in_off[c], a.idx, a.out_off[c], a.out_data[c], a.n);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -332,10 +355,10 @@ static Column gather_column_values(const CtxPtr& ctx, const Column& in, const ui
   a.n = n;
   const int64_t num_tiles = (n + GL_TILE - 1) / GL_TILE;
   {
-    a.sc = prepare_compact(ctx, num_tiles, resident_ctas(ctx, reinterpret_cast<const void*>(gather_lengths_scan_kernel), GA_THREADS), ctx->d_scalars + 1);
+    a.sc = prepare_compact(ctx, num_tiles, resident_ctas(ctx, reinterpret_cast<const void*>(gather_lengths_scan_kernel<false>), GA_THREADS), ctx->d_scalars + 1);
     {
       LaunchTimer lt(ctx, "gather_lengths_scan_kernel");
-      launch_compact(ctx, gather_lengths_scan_kernel, a.sc, a);
+      launch_compact(ctx, gather_lengths_scan_kernel<false>, a.sc, a);
     }
     FG_CUDA(cudaGetLastError());
     count_launch(ctx);
@@ -349,7 +372,7 @@ static Column gather_column_values(const CtxPtr& ctx, const Column& in, const ui
     int grid = stream_grid(ctx, (n + 31) / 32, GA_THREADS / 32);
     {
       LaunchTimer lt(ctx, "gather_utf8_copy_kernel");
-      gather_utf8_copy_kernel<<<grid, GA_THREADS, 0, ctx->stream>>>(static_cast<const uint8_t*>(in.values()), in.offs(), d_idx,
+      gather_utf8_copy_kernel<false><<<grid, GA_THREADS, 0, ctx->stream>>>(static_cast<const uint8_t*>(in.values()), in.offs(), d_idx,
                                                                   out.offsets->as<int32_t>(), out.data->as<uint8_t>(), n);
     }
     FG_CUDA(cudaGetLastError());
@@ -360,15 +383,76 @@ static Column gather_column_values(const CtxPtr& ctx, const Column& in, const ui
 
 // take() of several columns through one index vector: one launch for all fixed-width columns; the Utf8 columns' length
 // scans are launched back to back and their byte totals read with ONE host round trip (each used to cost its own).
-static std::vector<Column> gather_columns_values(const CtxPtr& ctx, const std::vector<const Column*>& in, const uint32_t* d_idx, int64_t n);
+// `pad` selects the PAD flavour of every kernel (see gather_fixed_multi_kernel); the launch labels say so, so a launch
+// profile tells the outer join's takes from the Inner join's.
+static std::vector<Column> gather_columns_values(const CtxPtr& ctx, const std::vector<const Column*>& in, const uint32_t* d_idx, int64_t n, bool pad);
 
-std::vector<Column> gather_columns(const CtxPtr& ctx, const std::vector<const Column*>& in, const uint32_t* d_idx, int64_t n) {
-  std::vector<Column> out = gather_columns_values(ctx, in, d_idx, n);
+// the validity of a padded take(): every column gets one (a padded row is NULL), one launch per column
+static void gather_validity_pad(const CtxPtr& ctx, const Column& in, Column& out, const uint32_t* d_idx, int64_t n) {
+  out.validity = alloc(ctx, size_t(n));
+  out.nullable = true;
+  if (n > 0) {
+    {
+      LaunchTimer lt(ctx, "gather_valid_pad_kernel");
+      gather_valid_pad_kernel<<<stream_grid(ctx, n, GA_THREADS * 4), GA_THREADS, 0, ctx->stream>>>(in.valid(), d_idx, out.validity->as<uint8_t>(), n);
+    }
+    FG_CUDA(cudaGetLastError());
+    count_launch(ctx);
+  }
+}
+
+std::vector<Column> null_columns(const CtxPtr& ctx, const Table& t, int64_t n) {
+  std::vector<Column> out(t.cols.size());
+  for (size_t k = 0; k < t.cols.size(); ++k) {
+    const Column& c = t.cols[k];
+    Column& o = out[k];
+    o.dtype = c.dtype;
+    o.name = c.name;
+    o.format = c.format;
+    o.nullable = true;
+    o.length = n;
+    o.validity = alloc(ctx, size_t(n));
+    if (n > 0) FG_CUDA(cudaMemsetAsync(o.validity->ptr, 0, size_t(n), ctx->stream));
+    if (c.dtype == FLOCKGPU_UTF8) {
+      o.offsets = alloc(ctx, size_t(n + 1) * 4);
+      FG_CUDA(cudaMemsetAsync(o.offsets->ptr, 0, size_t(n + 1) * 4, ctx->stream));
+      o.data = alloc(ctx, 0);
+      o.values_bytes = 0;
+    } else {
+      o.data = alloc(ctx, size_t(n) * c.width());
+      if (n > 0) FG_CUDA(cudaMemsetAsync(o.data->ptr, 0, size_t(n) * c.width(), ctx->stream));
+    }
+  }
+  return out;
+}
+
+std::vector<Column> gather_columns(const CtxPtr& ctx, const std::vector<const Column*>& in, const uint32_t* d_idx, int64_t n, bool pad) {
+  if (pad) {
+    // a column that is NULL as a whole (global aggregate over empty input) is NULL in every taken row too
+    std::vector<const Column*> live;
+    for (const Column* c : in)
+      if (!c->all_null) live.push_back(c);
+    std::vector<Column> got = gather_columns_values(ctx, live, d_idx, n, true);
+    std::vector<Column> out;
+    size_t g = 0;
+    for (const Column* c : in) {
+      if (c->all_null) {
+        Table one;
+        one.cols.push_back(*c);
+        out.push_back(std::move(null_columns(ctx, one, n)[0]));
+        continue;
+      }
+      gather_validity_pad(ctx, *c, got[g], d_idx, n);
+      out.push_back(std::move(got[g++]));
+    }
+    return out;
+  }
+  std::vector<Column> out = gather_columns_values(ctx, in, d_idx, n, false);
   for (size_t k = 0; k < in.size(); ++k) gather_validity(ctx, *in[k], out[k], d_idx, n);
   return out;
 }
 
-static std::vector<Column> gather_columns_values(const CtxPtr& ctx, const std::vector<const Column*>& in, const uint32_t* d_idx, int64_t n) {
+static std::vector<Column> gather_columns_values(const CtxPtr& ctx, const std::vector<const Column*>& in, const uint32_t* d_idx, int64_t n, bool pad) {
   std::vector<Column> out(in.size());
   std::vector<size_t> fixed, utf8;
   for (size_t k = 0; k < in.size(); ++k) {
@@ -382,6 +466,10 @@ static std::vector<Column> gather_columns_values(const CtxPtr& ctx, const std::v
     o.length = n;
     (c.dtype == FLOCKGPU_UTF8 ? utf8 : fixed).push_back(k);
   }
+  const auto lengths_scan = pad ? gather_lengths_scan_kernel<true> : gather_lengths_scan_kernel<false>;
+  const auto lengths_scan_multi = pad ? gather_lengths_scan_multi_kernel<true> : gather_lengths_scan_multi_kernel<false>;
+  const auto copy = pad ? gather_utf8_copy_kernel<true> : gather_utf8_copy_kernel<false>;
+  const auto copy_multi = pad ? gather_utf8_copy_multi_kernel<true> : gather_utf8_copy_multi_kernel<false>;
   for (size_t first = 0; first < fixed.size(); first += GM_MAX_COLS) {
     GatherMultiArgs a{};
     a.idx = d_idx;
@@ -397,8 +485,8 @@ static std::vector<Column> gather_columns_values(const CtxPtr& ctx, const std::v
     }
     if (n > 0) {
       {
-        LaunchTimer lt(ctx, "gather_fixed_multi_kernel");
-        gather_fixed_multi_kernel<<<stream_grid(ctx, n, GA_THREADS * 2), GA_THREADS, 0, ctx->stream>>>(a);
+        LaunchTimer lt(ctx, pad ? "gather_fixed_multi_kernel<PAD>" : "gather_fixed_multi_kernel");
+        (pad ? gather_fixed_multi_kernel<true> : gather_fixed_multi_kernel<false>)<<<stream_grid(ctx, n, GA_THREADS * 2), GA_THREADS, 0, ctx->stream>>>(a);
       }
       FG_CUDA(cudaGetLastError());
       count_launch(ctx);
@@ -410,7 +498,7 @@ static std::vector<Column> gather_columns_values(const CtxPtr& ctx, const std::v
   // byte totals, one copy launch (q3's join output takes name, city and state: 6 launches -> 2)
   if (n > 0 && utf8.size() >= 2 && utf8.size() <= size_t(GL_MAX_COLS) && ctx->compact_mode == 0) {
     const int64_t tiles = (n + GL_TILE - 1) / GL_TILE;
-    const int64_t resident = resident_ctas(ctx, reinterpret_cast<const void*>(gather_lengths_scan_multi_kernel), GA_THREADS);
+    const int64_t resident = resident_ctas(ctx, reinterpret_cast<const void*>(lengths_scan_multi), GA_THREADS);
     if (tiles * int64_t(utf8.size()) <= resident) {
       GatherLenMultiArgs la{};
       la.idx = d_idx;
@@ -427,8 +515,8 @@ static std::vector<Column> gather_columns_values(const CtxPtr& ctx, const std::v
       la.sc = prepare_compact(ctx, tiles * int64_t(utf8.size()), resident, ctx->d_scalars + kGatherTotalsSlot);
       if (la.sc.single_wave) {
         {
-          LaunchTimer lt(ctx, "gather_lengths_scan_multi_kernel");
-          launch_compact(ctx, gather_lengths_scan_multi_kernel, la.sc, la);
+          LaunchTimer lt(ctx, pad ? "gather_lengths_scan_multi_kernel<PAD>" : "gather_lengths_scan_multi_kernel");
+          launch_compact(ctx, lengths_scan_multi, la.sc, la);
         }
         FG_CUDA(cudaGetLastError());
         count_launch(ctx);
@@ -453,8 +541,8 @@ static std::vector<Column> gather_columns_values(const CtxPtr& ctx, const std::v
         if (any) {
           dim3 grid(unsigned(stream_grid(ctx, (n + 31) / 32, GA_THREADS / 32, 8 / int(utf8.size()) + 1)), unsigned(utf8.size()));
           {
-            LaunchTimer lt(ctx, "gather_utf8_copy_multi_kernel");
-            gather_utf8_copy_multi_kernel<<<grid, GA_THREADS, 0, ctx->stream>>>(ca);
+            LaunchTimer lt(ctx, pad ? "gather_utf8_copy_multi_kernel<PAD>" : "gather_utf8_copy_multi_kernel");
+            copy_multi<<<grid, GA_THREADS, 0, ctx->stream>>>(ca);
           }
           FG_CUDA(cudaGetLastError());
           count_launch(ctx);
@@ -480,10 +568,10 @@ static std::vector<Column> gather_columns_values(const CtxPtr& ctx, const std::v
     a.out_off = o.offsets->as<int32_t>();
     a.n = n;
     const int64_t num_tiles = (n + GL_TILE - 1) / GL_TILE;
-    a.sc = prepare_compact(ctx, num_tiles, resident_ctas(ctx, reinterpret_cast<const void*>(gather_lengths_scan_kernel), GA_THREADS), ctx->d_scalars + kGatherTotalsSlot + u);
+    a.sc = prepare_compact(ctx, num_tiles, resident_ctas(ctx, reinterpret_cast<const void*>(lengths_scan), GA_THREADS), ctx->d_scalars + kGatherTotalsSlot + u);
     {
-      LaunchTimer lt(ctx, "gather_lengths_scan_kernel");
-      launch_compact(ctx, gather_lengths_scan_kernel, a.sc, a);
+      LaunchTimer lt(ctx, pad ? "gather_lengths_scan_kernel<PAD>" : "gather_lengths_scan_kernel");
+      launch_compact(ctx, lengths_scan, a.sc, a);
     }
     FG_CUDA(cudaGetLastError());
     count_launch(ctx);
@@ -499,8 +587,8 @@ static std::vector<Column> gather_columns_values(const CtxPtr& ctx, const std::v
     o.data = alloc(ctx, size_t(totals[u]));
     if (totals[u] > 0) {
       {
-        LaunchTimer lt(ctx, "gather_utf8_copy_kernel");
-        gather_utf8_copy_kernel<<<stream_grid(ctx, (n + 31) / 32, GA_THREADS / 32), GA_THREADS, 0, ctx->stream>>>(
+        LaunchTimer lt(ctx, pad ? "gather_utf8_copy_kernel<PAD>" : "gather_utf8_copy_kernel");
+        copy<<<stream_grid(ctx, (n + 31) / 32, GA_THREADS / 32), GA_THREADS, 0, ctx->stream>>>(
             static_cast<const uint8_t*>(src.values()), src.offs(), d_idx, o.offsets->as<int32_t>(), o.data->as<uint8_t>(), n);
       }
       FG_CUDA(cudaGetLastError());

@@ -1,4 +1,4 @@
-// hash_join.cu -- K3/K4: HashJoinExec { mode: Partitioned, join_type: Inner }.
+// hash_join.cu -- K3/K4: HashJoinExec { mode: Partitioned, join_type: Inner | Left | Right | Full | Semi | Anti }.
 //
 // Reference operator (DataFusion fork, not in tree; used at flock/src/distributed_plan/planner.rs:169,
 // :239 and serialised in flock/src/tests/data/plan/join.json): build a hash map over ALL left batches
@@ -20,6 +20,21 @@
 //                            compaction over the probe side, no table
 // and gather.cu materialises the output columns (Utf8 included).  The kernels are instantiated per key shape:
 // one 4-byte key, one 8-byte key, or the general form (two packed columns / row comparison for Utf8 keys).
+//
+// The other join types keep the rule that the smaller input is hashed, so each has a form for its preserved (or
+// filtered) side being streamed and one for it being hashed:
+//   preserved side streamed   (Left with right hashed, Right with left hashed, Full): the count kernel counts
+//                             max(matches, 1) per probe row and the emit kernel writes the pad sentinel JOIN_EMPTY as
+//                             the build row of a row without a match -- the same two launches as Inner
+//   Semi / Anti, left streamed  join_filter_kernel: one stable compaction of the left rows, a row survives when its key
+//                             has a slot (Semi) or has none (Anti); no pairs, no chain walk
+//   preserved / filtered side hashed  (Left with left hashed, Right with right hashed, Full, Semi / Anti with left
+//                             hashed): visits are recorded PER SLOT -- the build pass stores each build row's slot, a
+//                             probe that finds a slot stores visited[slot] = 1 (idempotent, no atomics, no chain walk) --
+//                             and join_visited_kernel compacts the build rows whose slot was (Semi) or was not visited,
+//                             in build-row order.  Outer types append those rows after the pairs with the sentinel on
+//                             the probe side; for Semi / Anti they are the whole output.
+// A row with a NULL key has no slot: it matches nothing, is unvisited, and is kept by every type that keeps its side.
 #include <algorithm>
 
 #include "compact.cuh"
@@ -50,6 +65,8 @@ struct JoinTable {
   unsigned* next;          // [build rows] next build row with the same key, JOIN_EMPTY = end
   unsigned long long cap;  // power of two
   struct JoinSlot* slots;  // KW = 4: the table proper (below); rep / head / cnt are unused, `next` holds row + 1
+  unsigned* slot_of;       // [build rows] slot of the row's key, JOIN_EMPTY for a NULL key (hashed preserved side only)
+  uint8_t* visited;        // [cap] 1 = some probe row found this slot (hashed preserved side only)
 };
 
 // One 4-byte key (every NEXMark join but q5's): the KEY LIVES IN THE SLOT.  A probe is one 16-byte load -- key, list
@@ -103,10 +120,14 @@ __device__ __forceinline__ bool build_row_matches(const JoinSide& build, unsigne
   return build.packed ? pack_key(build.pack, build.cols, int64_t(r)) == key : rows_equal(build.rk, build.cols, int64_t(r), other.rk, other.cols, row);
 }
 
-template <int KW>
+// REC: also store each build row's slot in t.slot_of (the hashed side is preserved or filtered: join_visited_kernel)
+template <int KW, bool REC = false>
 __global__ void __launch_bounds__(256) join_build_kernel(const __grid_constant__ JoinSide build, const JoinTable t) {
   for (int64_t row = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; row < build.n_rows; row += int64_t(gridDim.x) * blockDim.x) {
-    if (key_is_null(build, row)) continue;  // never enters the table: nothing can match it
+    if (key_is_null(build, row)) {  // never enters the table: nothing can match it
+      if (REC) t.slot_of[row] = JOIN_EMPTY;
+      continue;
+    }
     unsigned long long key;
     unsigned long long slot = side_hash<KW>(build, row, &key) & (t.cap - 1);
     if (KW == 4) {
@@ -119,6 +140,7 @@ __global__ void __launch_bounds__(256) join_build_kernel(const __grid_constant__
       }
       t.next[row] = atomicExch(&t.slots[slot].head, unsigned(row) + 1u);
       atomicAdd(&t.slots[slot].cnt, 1u);
+      if (REC) t.slot_of[row] = unsigned(slot);
       continue;
     }
     while (true) {
@@ -132,6 +154,7 @@ __global__ void __launch_bounds__(256) join_build_kernel(const __grid_constant__
     }
     t.next[row] = atomicExch(&t.head[slot], unsigned(row));
     atomicAdd(&t.cnt[slot], 1u);
+    if (REC) t.slot_of[row] = unsigned(slot);
   }
 }
 
@@ -174,9 +197,14 @@ struct JoinCountArgs {
   JoinTable table;
   unsigned* out_off;  // [probe rows + 1] exclusive pair offsets
   CompactScratch sc;  // grid-wide exclusive prefix of the tiles' pair counts (compact.cuh); sc.out_count = total pairs
+  unsigned long long* pad_rows;  // JOIN_PAD_PROBE: receives the number of probe rows without a match (zeroed by the host)
 };
 
-template <int KW>
+// Forms of the count / emit kernels beyond Inner's (FORM = 0)
+constexpr int JOIN_PAD_PROBE = 1;  // the probe side is preserved: a probe row without a match yields one padded row
+constexpr int JOIN_MARK = 2;       // the build side is preserved: record visited[slot]
+
+template <int KW, int FORM = 0>
 __global__ void __launch_bounds__(JC_THREADS) join_count_scan_kernel(const __grid_constant__ JoinCountArgs a) {
   __shared__ CompactSmem<1, 16> sm;
   __shared__ unsigned long long s_warp[JC_THREADS / 32];
@@ -187,16 +215,28 @@ __global__ void __launch_bounds__(JC_THREADS) join_count_scan_kernel(const __gri
     const int64_t i0 = tile * JC_TILE + int64_t(tid) * JC_ITEMS;
     unsigned cnt[JC_ITEMS];
     unsigned long long local = 0;
+    unsigned pads = 0;
 #pragma unroll
     for (int k = 0; k < JC_ITEMS; ++k) {
       unsigned c = 0;
       if (i0 + k < n) {
         unsigned head = 0, in_slot = 0;
         const unsigned long long slot = find_slot<KW>(a.build, a.probe, a.table, i0 + k, &head, &in_slot);
-        if (slot != ~0ull) c = KW == 4 ? in_slot : a.table.cnt[slot];
+        if (slot != ~0ull) {
+          c = KW == 4 ? in_slot : a.table.cnt[slot];
+          if (FORM & JOIN_MARK) a.table.visited[slot] = 1;
+        }
+        if ((FORM & JOIN_PAD_PROBE) && c == 0) {
+          c = 1;
+          ++pads;
+        }
       }
       cnt[k] = c;
       local += c;
+    }
+    if (FORM & JOIN_PAD_PROBE) {
+      pads = warp_sum(pads);
+      if (lane == 0 && pads) atomicAdd(a.pad_rows, (unsigned long long)pads);
     }
     unsigned long long incl = warp_inclusive_sum(local);
     if (lane == 31) s_warp[warp] = incl;
@@ -293,13 +333,18 @@ struct JoinEmitArgs {
   unsigned* probe_idx;
 };
 
-template <int KW>
+template <int KW, int FORM = 0>
 __global__ void __launch_bounds__(256) join_emit_kernel(const __grid_constant__ JoinEmitArgs a) {
   for (int64_t row = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; row < a.probe.n_rows; row += int64_t(gridDim.x) * blockDim.x) {
     unsigned pos = a.off[row];
     if (a.off[row + 1] == pos) continue;
     unsigned head = 0, in_slot = 0;
     const unsigned long long slot = find_slot<KW>(a.build, a.probe, a.table, row, &head, &in_slot);
+    if ((FORM & JOIN_PAD_PROBE) && slot == ~0ull) {  // no match: one row, build side padded
+      a.build_idx[pos] = JOIN_EMPTY;
+      a.probe_idx[pos] = unsigned(row);
+      continue;
+    }
     if (KW == 4) {
       for (unsigned r1 = head; r1 != 0u; r1 = a.table.next[r1 - 1u]) {  // row + 1 links, 0 ends the list
         a.build_idx[pos] = r1 - 1u;
@@ -313,6 +358,73 @@ __global__ void __launch_bounds__(256) join_emit_kernel(const __grid_constant__ 
       a.probe_idx[pos] = unsigned(row);
       ++pos;
     }
+  }
+}
+
+// ---- Semi / Anti with the left side streamed, and the hashed side's (un)visited rows: one stable compaction each, on
+// the join_one_kernel skeleton.  Survivors are written in row order, so Semi / Anti keep the left input order.
+struct JoinSelectArgs {
+  CompactScratch sc;
+  JoinSide build, probe;  // join_filter_kernel: probe = the rows compacted
+  JoinTable table;
+  int64_t n_rows;         // rows compacted
+  unsigned* out_idx;
+};
+
+template <class Pred>
+__device__ __forceinline__ void join_select_rows(const JoinSelectArgs& a, Pred survives) {
+  constexpr int E = 4, I = 16, G = I / E;
+  constexpr int TILE = CP_THREADS * I;
+  __shared__ CompactSmem<E, I> sm;
+  const int tid = threadIdx.x;
+  long long tile;
+  for (int it = 0; (tile = cp_next_tile(sm, a.sc, it)) >= 0; ++it) {
+    const int64_t tile_base = tile * TILE;
+    unsigned long long bits = 0;
+#pragma unroll
+    for (int k = 0; k < I; ++k) {
+      const int64_t r = tile_base + cp_item_index<E>(k, tid);
+      if (r < a.n_rows && survives(r)) bits |= 1ull << k;
+    }
+    unsigned lane_prefix[G];
+    cp_rank_tile<E, I>(sm, a.sc, tile, bits, lane_prefix);
+    if (bits && sm.tile_total) {
+      unsigned long long m = bits;
+      while (m) {
+        const int k = __ffsll((long long)m) - 1;
+        m &= m - 1;
+        a.out_idx[cp_position<E, I>(sm, bits, k, lane_prefix)] = unsigned(tile_base + cp_item_index<E>(k, tid));
+      }
+    }
+    __syncthreads();
+  }
+}
+
+// left rows (streamed) whose key has a slot in the right side's table (Semi) or has none (Anti; a NULL key has none)
+template <int KW, bool ANTI>
+__global__ void __launch_bounds__(CP_THREADS) join_filter_kernel(const __grid_constant__ JoinSelectArgs a) {
+  join_select_rows(a, [&](int64_t r) {
+    unsigned head = 0, in_slot = 0;
+    return (find_slot<KW>(a.build, a.probe, a.table, r, &head, &in_slot) != ~0ull) != ANTI;
+  });
+}
+
+// build rows whose slot some probe row found (VISITED: Semi) or none did (outer types, Anti; a NULL key has no slot)
+template <bool VISITED>
+__global__ void __launch_bounds__(CP_THREADS) join_visited_kernel(const __grid_constant__ JoinSelectArgs a) {
+  join_select_rows(a, [&](int64_t r) {
+    const unsigned s = a.table.slot_of[r];
+    return (s != JOIN_EMPTY && a.table.visited[s]) == VISITED;
+  });
+}
+
+// every probe row that finds its key's slot marks it visited (Semi / Anti with the left side hashed: no pairs needed)
+template <int KW>
+__global__ void __launch_bounds__(256) join_mark_kernel(const __grid_constant__ JoinSide build, const __grid_constant__ JoinSide probe, const JoinTable t) {
+  for (int64_t row = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; row < probe.n_rows; row += int64_t(gridDim.x) * blockDim.x) {
+    unsigned head = 0, in_slot = 0;
+    const unsigned long long slot = find_slot<KW>(build, probe, t, row, &head, &in_slot);
+    if (slot != ~0ull) t.visited[slot] = 1;
   }
 }
 
@@ -348,13 +460,18 @@ static int grid_for(const CtxPtr& ctx, int64_t items, int threads, int per_sm) {
   return int(std::max<int64_t>(1, std::min<int64_t>((items + threads - 1) / threads, int64_t(ctx->sm_count) * per_sm)));
 }
 
+static TablePtr join_typed(const CtxPtr& ctx, const Table& L, const Table& R, const std::vector<int>& left_keys, const std::vector<int>& right_keys,
+                           const std::vector<int>& widths, bool packed, bool null_key, int join_type);
+
 TablePtr hash_join(const CtxPtr& ctx, const TablePtr& left_ptr, const TablePtr& right_ptr, const std::vector<int>& left_keys,
-                   const std::vector<int>& right_keys) {
+                   const std::vector<int>& right_keys, int join_type) {
+  FG_CHECK(join_type >= FLOCKGPU_JOIN_INNER && join_type <= FLOCKGPU_JOIN_ANTI, FLOCKGPU_ERR_INVALID, "hash_join: unknown join type %d", join_type);
   const Table& L = *left_ptr;
   const Table& R = *right_ptr;
   // one side is a single row and the other a group-by result still in table form (NEXMark q5: num = MAX(num)):
-  // an equality selection over the table, no rows are materialised for the join
-  if (left_keys.size() == 1 && right_keys.size() == 1) {
+  // an equality selection over the table, no rows are materialised for the join (Inner only: the other types take the
+  // general path below, which is correct for one-row and deferred inputs as they are)
+  if (join_type == FLOCKGPU_JOIN_INNER && left_keys.size() == 1 && right_keys.size() == 1) {
     if (std::shared_ptr<DeferredTable> d = left_ptr->deferred)
       if (TablePtr t = d->select_equal(L, left_keys[0], right_ptr, right_keys[0], true)) return t;
     if (std::shared_ptr<DeferredTable> d = right_ptr->deferred)
@@ -376,13 +493,14 @@ TablePtr hash_join(const CtxPtr& ctx, const TablePtr& left_ptr, const TablePtr& 
   }
   const bool packed = keys_packable(widths.data(), int(widths.size()));
 
-  auto out = std::make_shared<Table>();
-  out->ctx = ctx;
-  out->metadata = L.metadata;
-
   // a NULL key column (one-row global aggregate over empty input) matches nothing
   bool null_key = false;
   for (size_t i = 0; i < left_keys.size(); ++i) null_key |= L.cols[left_keys[i]].all_null || R.cols[right_keys[i]].all_null;
+  if (join_type != FLOCKGPU_JOIN_INNER) return join_typed(ctx, L, R, left_keys, right_keys, widths, packed, null_key, join_type);
+
+  auto out = std::make_shared<Table>();
+  out->ctx = ctx;
+  out->metadata = L.metadata;
 
   int64_t n_pairs = 0;
   BufferPtr build_idx, probe_idx;
@@ -449,7 +567,7 @@ TablePtr hash_join(const CtxPtr& ctx, const TablePtr& left_ptr, const TablePtr& 
       FG_CUDA(cudaMemsetAsync(tbuf->ptr, 0xff, size_t(cap) * 8, ctx->stream));                                  // rep, head = EMPTY
       FG_CUDA(cudaMemsetAsync(static_cast<char*>(tbuf->ptr) + size_t(cap) * 8, 0, size_t(cap) * 4, ctx->stream));  // cnt = 0
       unsigned* w = tbuf->as<unsigned>();
-      tab = JoinTable{w, w + cap, w + 2 * cap, w + 3 * cap, cap, nullptr};
+      tab = JoinTable{w, w + cap, w + 2 * cap, w + 3 * cap, cap, nullptr, nullptr, nullptr};
     }
     {
       LaunchTimer lt(ctx, "join_build_kernel");
@@ -514,6 +632,221 @@ TablePtr hash_join(const CtxPtr& ctx, const TablePtr& left_ptr, const TablePtr& 
   return out;
 }
 
+
+// ---- Left / Right / Full / Semi / Anti ------------------------------------------------------------------------------
+static TablePtr join_typed(const CtxPtr& ctx, const Table& L, const Table& R, const std::vector<int>& left_keys, const std::vector<int>& right_keys,
+                           const std::vector<int>& widths, bool packed, bool null_key, int join_type) {
+  const bool semi_anti = join_type == FLOCKGPU_JOIN_SEMI || join_type == FLOCKGPU_JOIN_ANTI;
+  const bool keep_left = join_type == FLOCKGPU_JOIN_LEFT || join_type == FLOCKGPU_JOIN_FULL;   // unmatched left rows are kept
+  const bool keep_right = join_type == FLOCKGPU_JOIN_RIGHT || join_type == FLOCKGPU_JOIN_FULL;
+  // output: left ++ right (left only for Semi / Anti); the side that can be padded is nullable whatever the data
+  auto assemble = [&](std::vector<Column> lcols, std::vector<Column> rcols, int64_t rows) {
+    auto out = std::make_shared<Table>();
+    out->ctx = ctx;
+    out->metadata = L.metadata;
+    out->num_rows = rows;
+    for (Column& c : lcols) {
+      c.nullable |= keep_right;
+      out->cols.push_back(std::move(c));
+    }
+    if (!semi_anti)
+      for (Column& c : rcols) {
+        c.nullable |= keep_left;
+        out->cols.push_back(std::move(c));
+      }
+    return TablePtr(out);
+  };
+
+  if (L.num_rows == 0 || R.num_rows == 0 || null_key) {
+    // nothing matches: the preserved side(s) padded, no kernel
+    switch (join_type) {
+      case FLOCKGPU_JOIN_SEMI: return assemble(empty_like(ctx, L)->cols, {}, 0);
+      case FLOCKGPU_JOIN_ANTI: return assemble(L.cols, {}, L.num_rows);
+      case FLOCKGPU_JOIN_LEFT: return assemble(L.cols, null_columns(ctx, R, L.num_rows), L.num_rows);
+      case FLOCKGPU_JOIN_RIGHT: return assemble(null_columns(ctx, L, R.num_rows), R.cols, R.num_rows);
+      default: {
+        TablePtr lpart = assemble(L.cols, null_columns(ctx, R, L.num_rows), L.num_rows);
+        TablePtr rpart = assemble(null_columns(ctx, L, R.num_rows), R.cols, R.num_rows);
+        if (R.num_rows == 0) return lpart;
+        if (L.num_rows == 0) return rpart;
+        return concat_tables(ctx, {lpart, rpart});
+      }
+    }
+  }
+
+  // hash the smaller input, stream the larger one through it (as Inner)
+  const bool swap_sides = R.num_rows < L.num_rows;
+  const Table& B = swap_sides ? R : L;
+  const Table& P = swap_sides ? L : R;
+  // the hashed side needs visit records when its unmatched rows are output (outer) or it is the side Semi / Anti filter
+  const bool keep_build = semi_anti ? !swap_sides : (swap_sides ? keep_right : keep_left);
+  const bool keep_probe = !semi_anti && (swap_sides ? keep_left : keep_right);
+  JoinSide bs{}, ps{};
+  fill_side(B, swap_sides ? right_keys : left_keys, packed, &bs);
+  fill_side(P, swap_sides ? left_keys : right_keys, packed, &ps);
+  const int kw = (packed && widths.size() == 1) ? widths[0] : 0;
+  if (kw) {
+    bs.key0 = B.cols[(swap_sides ? right_keys : left_keys)[0]].values();
+    ps.key0 = P.cols[(swap_sides ? left_keys : right_keys)[0]].values();
+  }
+  auto by_width = [&](auto&& f) {
+    if (kw == 4) f(std::integral_constant<int, 4>{});
+    else if (kw == 8) f(std::integral_constant<int, 8>{});
+    else f(std::integral_constant<int, 0>{});
+  };
+
+  unsigned long long cap = 1024;
+  while (cap < 2ull * (unsigned long long)B.num_rows) cap <<= 1;
+  FG_CHECK(cap < (1ull << 32), FLOCKGPU_ERR_UNSUPPORTED, "hash_join: %lld build rows exceed the typed join's slot range", (long long)B.num_rows);
+  const size_t slots_bytes = kw == 4 ? size_t(cap) * sizeof(JoinSlot) : size_t(cap) * 12;
+  const size_t next_bytes = size_t(B.num_rows) * 4;
+  const size_t visit_bytes = keep_build ? next_bytes + size_t(cap) : 0;  // slot_of[build rows], visited[cap]
+  BufferPtr tbuf = alloc(ctx, slots_bytes + next_bytes + visit_bytes);
+  JoinTable tab{};
+  if (kw == 4) {
+    FG_CUDA(cudaMemsetAsync(tbuf->ptr, 0, slots_bytes, ctx->stream));
+    tab.slots = tbuf->as<JoinSlot>();
+    tab.next = reinterpret_cast<unsigned*>(tab.slots + cap);
+    tab.cap = cap;
+  } else {
+    FG_CUDA(cudaMemsetAsync(tbuf->ptr, 0xff, size_t(cap) * 8, ctx->stream));
+    FG_CUDA(cudaMemsetAsync(static_cast<char*>(tbuf->ptr) + size_t(cap) * 8, 0, size_t(cap) * 4, ctx->stream));
+    unsigned* w = tbuf->as<unsigned>();
+    tab = JoinTable{w, w + cap, w + 2 * cap, w + 3 * cap, cap, nullptr, nullptr, nullptr};
+  }
+  if (keep_build) {
+    tab.slot_of = reinterpret_cast<unsigned*>(static_cast<char*>(tbuf->ptr) + slots_bytes + next_bytes);
+    tab.visited = reinterpret_cast<uint8_t*>(tab.slot_of + B.num_rows);
+    FG_CUDA(cudaMemsetAsync(tab.visited, 0, size_t(cap), ctx->stream));
+  }
+  {
+    LaunchTimer lt(ctx, keep_build ? "join_build_kernel<REC>" : "join_build_kernel");
+    by_width([&](auto w) {
+      constexpr int KW = decltype(w)::value;
+      (keep_build ? join_build_kernel<KW, true> : join_build_kernel<KW, false>)<<<grid_for(ctx, B.num_rows, 256, 8), 256, 0, ctx->stream>>>(bs, tab);
+    });
+  }
+  FG_CUDA(cudaGetLastError());
+  count_launch(ctx);
+
+  // one stable compaction (join_filter_kernel / join_visited_kernel) of `n` rows into `out_idx`, its count to d_scalars[slot]
+  auto select = [&](auto kernel, const char* label, int64_t n, unsigned* out_idx, int slot) {
+    JoinSelectArgs sa{};
+    sa.build = bs;
+    sa.probe = ps;
+    sa.table = tab;
+    sa.n_rows = n;
+    sa.out_idx = out_idx;
+    const int64_t num_tiles = (n + CP_THREADS * 16 - 1) / (CP_THREADS * 16);
+    sa.sc = prepare_compact(ctx, num_tiles, resident_ctas(ctx, reinterpret_cast<const void*>(kernel), CP_THREADS), ctx->d_scalars + slot);
+    {
+      LaunchTimer lt(ctx, label);
+      launch_compact(ctx, kernel, sa.sc, sa);
+    }
+    FG_CUDA(cudaGetLastError());
+    count_launch(ctx);
+  };
+
+  if (semi_anti) {
+    // left rows, in left order, through one index vector
+    const bool anti = join_type == FLOCKGPU_JOIN_ANTI;
+    BufferPtr idx = alloc(ctx, size_t(L.num_rows) * 4);
+    if (swap_sides) {
+      // left streamed: a row survives on whether its key has a slot
+      by_width([&](auto w) {
+        constexpr int KW = decltype(w)::value;
+        select(anti ? join_filter_kernel<KW, true> : join_filter_kernel<KW, false>, anti ? "join_filter_kernel<ANTI>" : "join_filter_kernel<SEMI>",
+               L.num_rows, idx->as<unsigned>(), 4);
+      });
+    } else {
+      // left hashed: the right rows mark the slots they find, then the left rows are selected on their slot's mark
+      {
+        LaunchTimer lt(ctx, "join_mark_kernel");
+        by_width([&](auto w) { join_mark_kernel<decltype(w)::value><<<grid_for(ctx, P.num_rows, 256, 8), 256, 0, ctx->stream>>>(bs, ps, tab); });
+      }
+      FG_CUDA(cudaGetLastError());
+      count_launch(ctx);
+      select(anti ? join_visited_kernel<false> : join_visited_kernel<true>, anti ? "join_visited_kernel<UNVISITED>" : "join_visited_kernel<VISITED>",
+             L.num_rows, idx->as<unsigned>(), 4);
+    }
+    unsigned long long total = 0;
+    read_scalars(ctx, 4, 1, &total);
+    FG_CHECK(total <= (unsigned long long)L.num_rows, FLOCKGPU_ERR_CUDA, "hash_join: corrupt row count");
+    if (total == 0) return assemble(empty_like(ctx, L)->cols, {}, 0);
+    std::vector<const Column*> lsrc;
+    for (const Column& c : L.cols) lsrc.push_back(&c);
+    return assemble(gather_columns(ctx, lsrc, idx->as<uint32_t>(), int64_t(total)), {}, int64_t(total));
+  }
+
+  // ---- outer: pairs (+ one padded row per unmatched probe row), then the unmatched build rows
+  BufferPtr off = alloc(ctx, size_t(P.num_rows + 1) * 4);
+  if (keep_probe) FG_CUDA(cudaMemsetAsync(ctx->d_scalars + 6, 0, 8, ctx->stream));
+  JoinCountArgs ca{};
+  ca.build = bs;
+  ca.probe = ps;
+  ca.table = tab;
+  ca.out_off = off->as<unsigned>();
+  ca.pad_rows = ctx->d_scalars + 6;
+  const int64_t num_tiles = (P.num_rows + JC_TILE - 1) / JC_TILE;
+  auto count_form = [&](auto w, auto form) {
+    auto kernel = join_count_scan_kernel<decltype(w)::value, decltype(form)::value>;
+    ca.sc = prepare_compact(ctx, num_tiles, resident_ctas(ctx, reinterpret_cast<const void*>(kernel), JC_THREADS), ctx->d_scalars + 4);
+    LaunchTimer lt(ctx, keep_probe ? (keep_build ? "join_count_scan_kernel<PAD,MARK>" : "join_count_scan_kernel<PAD>") : "join_count_scan_kernel<MARK>");
+    launch_compact(ctx, kernel, ca.sc, ca);
+  };
+  by_width([&](auto w) {
+    if (keep_probe && keep_build) count_form(w, std::integral_constant<int, JOIN_PAD_PROBE | JOIN_MARK>{});
+    else if (keep_probe) count_form(w, std::integral_constant<int, JOIN_PAD_PROBE>{});
+    else count_form(w, std::integral_constant<int, JOIN_MARK>{});
+  });
+  FG_CUDA(cudaGetLastError());
+  count_launch(ctx);
+  BufferPtr unvisited;
+  if (keep_build) {
+    unvisited = alloc(ctx, size_t(B.num_rows) * 4);
+    select(join_visited_kernel<false>, "join_visited_kernel<UNVISITED>", B.num_rows, unvisited->as<unsigned>(), 5);
+  }
+  unsigned long long sc3[3] = {0, 0, 0};  // pairs incl. padded probe rows, unmatched build rows, padded probe rows
+  read_scalars(ctx, 4, 3, sc3);
+  const unsigned long long n_unvisited = keep_build ? sc3[1] : 0, n_pad_probe = keep_probe ? sc3[2] : 0;
+  FG_CHECK(n_unvisited <= (unsigned long long)B.num_rows && n_pad_probe <= (unsigned long long)P.num_rows, FLOCKGPU_ERR_CUDA, "hash_join: corrupt row count");
+  FG_CHECK(sc3[0] + n_unvisited < (1ull << 32) - 1, FLOCKGPU_ERR_UNSUPPORTED, "hash_join: %llu output rows exceed 2^32-2", sc3[0] + n_unvisited);
+  const int64_t n_pairs = int64_t(sc3[0]), n_rows = n_pairs + int64_t(n_unvisited);
+  BufferPtr build_idx = alloc(ctx, size_t(n_rows) * 4), probe_idx = alloc(ctx, size_t(n_rows) * 4);
+  if (n_pairs > 0) {
+    JoinEmitArgs ea{};
+    ea.build = bs;
+    ea.probe = ps;
+    ea.table = tab;
+    ea.off = off->as<unsigned>();
+    ea.build_idx = build_idx->as<unsigned>();
+    ea.probe_idx = probe_idx->as<unsigned>();
+    {
+      LaunchTimer lt(ctx, keep_probe ? "join_emit_kernel<PAD>" : "join_emit_kernel");
+      by_width([&](auto w) {
+        constexpr int KW = decltype(w)::value;
+        (keep_probe ? join_emit_kernel<KW, JOIN_PAD_PROBE> : join_emit_kernel<KW, 0>)<<<grid_for(ctx, P.num_rows, 256, 8), 256, 0, ctx->stream>>>(ea);
+      });
+    }
+    FG_CUDA(cudaGetLastError());
+    count_launch(ctx);
+  }
+  if (n_unvisited > 0) {
+    FG_CUDA(cudaMemcpyAsync(build_idx->as<unsigned>() + n_pairs, unvisited->ptr, size_t(n_unvisited) * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+    FG_CUDA(cudaMemsetAsync(probe_idx->as<unsigned>() + n_pairs, 0xff, size_t(n_unvisited) * 4, ctx->stream));  // JOIN_EMPTY
+  }
+  // sentinels in build_idx: the padded probe rows; in probe_idx: the unmatched build rows
+  const uint32_t* l_idx = (swap_sides ? probe_idx : build_idx)->as<uint32_t>();
+  const uint32_t* r_idx = (swap_sides ? build_idx : probe_idx)->as<uint32_t>();
+  const bool l_pad = (swap_sides ? n_unvisited : n_pad_probe) > 0, r_pad = (swap_sides ? n_pad_probe : n_unvisited) > 0;
+  std::vector<const Column*> lsrc, rsrc;
+  for (const Column& c : L.cols) lsrc.push_back(&c);
+  for (const Column& c : R.cols) rsrc.push_back(&c);
+  std::vector<Column> lcols = gather_columns(ctx, lsrc, l_idx, n_rows, l_pad);
+  std::vector<Column> rcols = gather_columns(ctx, rsrc, r_idx, n_rows, r_pad);
+  return assemble(std::move(lcols), std::move(rcols), n_rows);
+}
+
 }  // namespace fg
 
 using namespace fg;
@@ -528,5 +861,19 @@ extern "C" int flockgpu_hash_join(flockgpu_ctx* ctx, const flockgpu_table* left,
     FG_CUDA(cudaSetDevice(c->device));
     std::vector<int> lk(left_keys, left_keys + n_keys), rk(right_keys, right_keys + n_keys);
     *out = wrap_table(hash_join(c, left->table, right->table, lk, rk));
+  });
+}
+
+extern "C" int flockgpu_hash_join_typed(flockgpu_ctx* ctx, const flockgpu_table* left, const flockgpu_table* right, const int32_t* left_keys,
+                                        const int32_t* right_keys, int32_t n_keys, int32_t join_type, flockgpu_table** out) {
+  return guarded([&] {
+    auto c = core_of(ctx);
+    FG_CHECK(out && left && left->table && right && right->table && left_keys && right_keys && n_keys > 0, FLOCKGPU_ERR_INVALID,
+             "hash_join: null or empty argument");
+    FG_CHECK(join_type >= FLOCKGPU_JOIN_INNER && join_type <= FLOCKGPU_JOIN_ANTI, FLOCKGPU_ERR_INVALID, "hash_join: unknown join type %d", join_type);
+    std::lock_guard<std::recursive_mutex> g(c->mu);
+    FG_CUDA(cudaSetDevice(c->device));
+    std::vector<int> lk(left_keys, left_keys + n_keys), rk(right_keys, right_keys + n_keys);
+    *out = wrap_table(hash_join(c, left->table, right->table, lk, rk, join_type));
   });
 }

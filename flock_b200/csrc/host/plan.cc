@@ -492,13 +492,22 @@ TablePtr HashAggregateExec::execute_uncached(const ExecEnv& env) {
   return rename_columns(env, out, names);
 }
 
+// DataFusion 6 JoinType names, in the order of enum flockgpu_join_type
+static const char* const kJoinTypeNames[] = {"Inner", "Left", "Right", "Full", "Semi", "Anti"};
+
 std::string HashJoinExec::fmt_as() const {
-  std::string s = "HashJoinExec: mode=" + mode + ", join_type=Inner, on=[";
+  std::string s = "HashJoinExec: mode=" + mode + ", join_type=" + kJoinTypeNames[join_type] + ", on=[";
   for (size_t i = 0; i < on.size(); ++i) s += std::string(i ? ", " : "") + "(" + on[i].first.name + ", " + on[i].second.name + ")";
   return s + "]";
 }
 
 TablePtr HashJoinExec::execute(const ExecEnv& env) {
+  // Across GPUs only a Partitioned join (the exchange brought each key's rows to one rank) may emit unmatched left rows:
+  // with CollectLeft every rank holds the whole left side and each would emit its unmatched rows again.
+  const bool keeps_left_rows = join_type == FLOCKGPU_JOIN_LEFT || join_type == FLOCKGPU_JOIN_FULL || join_type == FLOCKGPU_JOIN_SEMI ||
+                               join_type == FLOCKGPU_JOIN_ANTI;
+  if (env.world > 1 && keeps_left_rows && mode != "Partitioned")
+    fail(FLOCKGPU_ERR_UNSUPPORTED, "HashJoinExec: join_type=%s in mode %s is not supported across GPUs (Partitioned only)", kJoinTypeNames[join_type], mode.c_str());
   TablePtr l = left->execute(env);
   TablePtr r = right->execute(env);
   std::vector<int> lk, rk;
@@ -506,7 +515,7 @@ TablePtr HashJoinExec::execute(const ExecEnv& env) {
     lk.push_back(resolve_column(*l, p.first.name, p.first.index));
     rk.push_back(resolve_column(*r, p.second.name, p.second.index));
   }
-  return fg::hash_join(env.ctx, l, r, lk, rk);
+  return fg::hash_join(env.ctx, l, r, lk, rk, join_type);
 }
 
 std::string SortExec::fmt_as() const {
@@ -654,7 +663,10 @@ static PlanPtr build_plan(const Json& j) {
   if (tag == "hash_join_exec") {
     auto n = std::make_shared<HashJoinExec>();
     const std::string& jt = j.at("join_type").as_string("join_type");
-    if (jt != "Inner") fail(FLOCKGPU_ERR_UNSUPPORTED, "plan: join_type %s is not supported on the GPU path (Inner only)", jt.c_str());
+    n->join_type = -1;
+    for (int t = FLOCKGPU_JOIN_INNER; t <= FLOCKGPU_JOIN_ANTI; ++t)
+      if (jt == kJoinTypeNames[t]) n->join_type = t;
+    if (n->join_type < 0) fail(FLOCKGPU_ERR_INVALID, "plan JSON: unknown join_type %s", jt.c_str());
     if (const Json* m = j.get("mode")) n->mode = m->is_string() ? m->str : "Partitioned";
     for (const JsonPtr& pair : j.at("on").arr) {
       if (!pair->is_array() || pair->arr.size() != 2) fail(FLOCKGPU_ERR_INVALID, "plan JSON: join `on` entries must be pairs");

@@ -148,6 +148,7 @@ class HashJoinExec : public ExecutionPlan {
   };
   std::vector<std::pair<OnCol, OnCol>> on;
   std::string mode = "Partitioned";
+  int join_type = FLOCKGPU_JOIN_INNER;  // DataFusion 6 JoinType; "Inner" ... "Anti" in the plan JSON
   const char* name() const override { return "HashJoinExec"; }
   std::vector<PlanPtr> children() const override { return {left, right}; }
   std::string fmt_as() const override;

@@ -431,7 +431,8 @@ TablePtr hash_aggregate(const CtxPtr& ctx, const TablePtr& in, int mode, const s
 // Estimate from the first 64 Ki rows: fraction of rows that repeat an earlier group key (hash_agg.cu).
 double distinct_sample_duplicates(const CtxPtr& ctx, const TablePtr& in, const std::vector<int>& group_cols);
 TablePtr hash_join(const CtxPtr& ctx, const TablePtr& left, const TablePtr& right,
-                   const std::vector<int>& left_keys, const std::vector<int>& right_keys);
+                   const std::vector<int>& left_keys, const std::vector<int>& right_keys,
+                   int join_type = FLOCKGPU_JOIN_INNER);
 std::vector<TablePtr> hash_partition(const CtxPtr& ctx, const TablePtr& in, const std::vector<int>& keys,
                                      int n_parts);
 // The columns of `keys` that actually route a row: the fixed-width ones when there are any (hashing `p_id` routes
@@ -456,7 +457,12 @@ TablePtr gather_rows(const CtxPtr& ctx, const Table& in, const std::vector<int>&
                      int64_t n_idx);
 // Gathers single columns (used by filter for Utf8 pass-through and by join).
 Column gather_column(const CtxPtr& ctx, const Column& in, const uint32_t* d_idx, int64_t n_idx);
-std::vector<Column> gather_columns(const CtxPtr& ctx, const std::vector<const Column*>& in, const uint32_t* d_idx, int64_t n);
+// `pad`: d_idx may hold the pad sentinel ~0u (the unmatched rows of an outer join): such a row is NULL -- value 0,
+// Utf8 length 0, validity 0 -- and every output column carries validity bytes.
+std::vector<Column> gather_columns(const CtxPtr& ctx, const std::vector<const Column*>& in, const uint32_t* d_idx, int64_t n, bool pad = false);
+// `n` rows of NULL in the columns of `t` (validity 0, values 0, Utf8 empty), marked nullable: the padded side of an
+// outer join whose other side found no partner at all.
+std::vector<Column> null_columns(const CtxPtr& ctx, const Table& t, int64_t n);
 
 TablePtr all_to_all(const CtxPtr& ctx, const std::vector<TablePtr>& parts);
 void comm_unique_id(uint8_t* out);

@@ -97,8 +97,9 @@ def hash_aggregate_exec(mode: str, group_expr: list[tuple[dict, str]], aggr_expr
             "aggr_expr": aggr_expr, "input": input}
 
 
-def hash_join_exec(left: dict, right: dict, on: list[tuple[dict, dict]], mode: str = "Partitioned") -> dict:
-    return {"execution_plan": "hash_join_exec", "join_type": "Inner", "mode": mode, "left": left, "right": right,
+def hash_join_exec(left: dict, right: dict, on: list[tuple[dict, dict]], mode: str = "Partitioned", join_type: str = "Inner") -> dict:
+    """join_type: DataFusion 6 JoinType -- Inner, Left, Right, Full, Semi or Anti."""
+    return {"execution_plan": "hash_join_exec", "join_type": join_type, "mode": mode, "left": left, "right": right,
             "on": [[{"name": l["name"], "index": l["index"]}, {"name": r["name"], "index": r["index"]}] for l, r in on]}
 
 

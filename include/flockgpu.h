@@ -277,13 +277,31 @@ int flockgpu_hash_aggregate(flockgpu_ctx* ctx, const flockgpu_table* in, int32_t
                             const int32_t* group_cols, int32_t n_group_cols,
                             const flockgpu_agg_spec* aggs, int32_t n_aggs, flockgpu_table** out);
 
-/* ---- HashJoinExec { mode: Partitioned, join_type: Inner } (planner.rs:169, :239) ---------------
- * out = left ++ right columns for every pair with equal keys (NULL != NULL; duplicates give the
- * full cross product).  `left` is the build side, exactly as in the reference (the textual left of
- * the SQL join).  Key column types must match pairwise (Int32/Int64/UInt64/Timestamp/Utf8).        */
+/* ---- HashJoinExec { mode: Partitioned, join_type: Inner | Left | Right | Full | Semi | Anti } (planner.rs:169, :239)
+ * Inner: out = left ++ right columns for every pair with equal keys (NULL != NULL; duplicates give the
+ * full cross product).  `left` is the textual left of the SQL join, as in the reference.  Key column
+ * types must match pairwise (Int32/Int64/UInt64/Timestamp/Utf8).
+ * The other DataFusion 6 join types (flockgpu_hash_join_typed):
+ *   Left   left ++ right: every pair, plus each left row without a match, its right columns NULL
+ *   Right  left ++ right: every pair, plus each right row without a match, its left columns NULL
+ *   Full   Left and Right together: pairs, unmatched left rows, unmatched right rows
+ *   Semi   left columns only: each left row with at least one match, once, in left input order
+ *   Anti   left columns only: each left row without a match, in left input order
+ * A row whose key is NULL matches nothing but is still a row of its side (kept by Left / Right / Full,
+ * returned by Anti).  The padded side's columns are nullable in the output; a padded value is NULL
+ * (fixed width 0, Utf8 empty).  Row order of Inner / Left / Right / Full is unspecified.           */
+enum flockgpu_join_type {
+  FLOCKGPU_JOIN_INNER = 0, FLOCKGPU_JOIN_LEFT = 1, FLOCKGPU_JOIN_RIGHT = 2, FLOCKGPU_JOIN_FULL = 3,
+  FLOCKGPU_JOIN_SEMI = 4, FLOCKGPU_JOIN_ANTI = 5
+};
+/* Inner join; the same as flockgpu_hash_join_typed(..., FLOCKGPU_JOIN_INNER, out). */
 int flockgpu_hash_join(flockgpu_ctx* ctx, const flockgpu_table* left, const flockgpu_table* right,
                        const int32_t* left_keys, const int32_t* right_keys, int32_t n_keys,
                        flockgpu_table** out);
+/* Any join type; an unknown `join_type` is FLOCKGPU_ERR_INVALID. */
+int flockgpu_hash_join_typed(flockgpu_ctx* ctx, const flockgpu_table* left, const flockgpu_table* right,
+                             const int32_t* left_keys, const int32_t* right_keys, int32_t n_keys,
+                             int32_t join_type, flockgpu_table** out);
 
 /* ---- SortExec / WindowAggExec(ROW_NUMBER) / GlobalLimitExec: what NEXMark q6 adds (benchmarks/src/nexmark/query/
  *      q6.sql, q6_plan.fmt; serialised sort_exec / global_limit_exec: flock/src/tests/data/plan/join.json) ------------- */
